@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — SVD UNet train-step frames/sec on B200 (BASELINE.json metric), one JSON line on rank 0.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|4|5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|4|5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -63,7 +63,16 @@ def parse():
     ap.add_argument("--no-script-path", action="store_true", help="skip the unchanged-script (eager, torch.optim.AdamW) timing")
     ap.add_argument("--no-graph", action="store_true", help="do not capture the step in a CUDA graph")
     ap.add_argument("--profile-one", action="store_true", help="run warm-up + one eager step only (for ncu)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed to DIR/<name>.npy: the UNet prediction, "
+                         "the loss, and a fixed seeded sample of the updated trainable weights and of their gradients (float32), "
+                         "with the sample positions (float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 def peaks():
@@ -317,6 +326,30 @@ def _emit(saved_fd, line):
     os.write(saved_fd, (json.dumps(line) + "\n").encode())
 
 
+DUMP_SAMPLE = 1 << 20      # sampled elements of the trainable weights and of their gradients (4 MB each in float32)
+
+
+def dump_outputs(out_dir, pred, loss, params):
+    """What the last timed step hands its caller, as out_dir/<name>.npy in float32: `pred` (the UNet output), `loss`, and
+    the updated weights and the gradients of the trainable parameters, flattened in parameter order, at DUMP_SAMPLE
+    positions drawn with a fixed seed (`weights_sample`, `grads_sample`; the positions in `sample_index`, float64).
+    Two runs with the same arguments agree to the bf16 noise floor, not bitwise: the GroupNorm statistics use fp32 atomics
+    (DESIGN.md, run-to-run reproducibility)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(p.numel() for p in params)
+    if total > DUMP_SAMPLE:
+        idx = torch.randint(total, (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).unique()
+    else:
+        idx = torch.arange(total)
+    dev_idx = idx.to(params[0].device)
+    weights = torch.cat([p.detach().reshape(-1) for p in params])[dev_idx]
+    grads = torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).reshape(-1) for p in params])[dev_idx]
+    for name, t in (("pred", pred), ("loss", loss), ("weights_sample", weights), ("grads_sample", grads)):
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+    np.save(os.path.join(out_dir, "sample_index.npy"), idx.double().numpy())
+
+
 def main():
     args = parse()
     out_fd = _protect_stdout()
@@ -409,7 +442,7 @@ def main():
         if reducer is not None:
             reducer.finish()
         opt.step()
-        return loss
+        return loss, pred
 
     def barrier():
         if world > 1:
@@ -480,12 +513,14 @@ def main():
     c0 = clocks.count() if clocks is not None else 0
     e0.record()
     for _ in range(args.steps):
-        loss = run_step()
+        loss, pred = run_step()
     e1.record()
     barrier()
     c1 = clocks.count() if clocks is not None else 0
     ms = e0.elapsed_time(e1)
     launches = raw.LAUNCHES[0] - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, pred, loss, [p for p in unet.parameters() if p.requires_grad])
     for _ in range(2):          # one more sampling period under load before the sampler stops
         run_step()
     torch.cuda.synchronize()
@@ -501,9 +536,9 @@ def main():
     # ---- e2e: public API from pinned host buffers, H2D inside, loss read back every step
     def e2e_step():
         if graphed is not None:     # pinned host -> static device buffers -> one graph launch -> loss back to the host
-            return float(graphed(host).item())
+            return float(graphed(host)[0].item())
         b = {k: v.to(dev, non_blocking=True) for k, v in host.items()}
-        return float(step(b).item())
+        return float(step(b)[0].item())
 
     e2e_step()
     barrier()

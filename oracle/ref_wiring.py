@@ -11,8 +11,8 @@ statement of it, on identical blocks: constructor channel bookkeeping, state-dic
 repeat / skip-connection order, the plugin API. What it does NOT pin: the arithmetic inside the blocks, which both
 sides take from the oracle (that part stays "parity unpinned" against diffusers — see oracle/svd_unet_oracle.py).
 
-Used by tests/golden/make_ref_wiring_golden.py (writes the committed fixture) and, when /root/reference exists, by
-tests/test_reference_wiring.py for a live A/B. Nothing here is imported by the product path.
+Used by tests/golden/make_ref_wiring_golden.py, which writes the committed fixture that tests/test_reference_wiring.py
+checks the oracle against. Nothing here is imported by the product path.
 """
 from __future__ import annotations
 
@@ -127,7 +127,7 @@ def _stubbed_diffusers():
                 sys.modules[k] = v
 
 
-def load_reference_unet_class(reference_root: str = "/root/reference"):
+def load_reference_unet_class(reference_root: str):
     """import <reference_root>/src/unet_spatio_temporal_condition.py (unmodified, from where it lies) over the stand-in
     diffusers namespace and return its UNetSpatioTemporalConditionModel class"""
     path = os.path.join(reference_root, REFERENCE_FILE)

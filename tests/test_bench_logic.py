@@ -77,6 +77,29 @@ def test_clock_sampler_brackets_the_timed_region(bench, tmp_path, monkeypatch):
     assert out["samples"] == 3 and "hw_slowdown" in out["reasons"]
 
 
+def test_dump_outputs_writes_a_fixed_sample(bench, tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    monkeypatch.setattr(bench, "DUMP_SAMPLE", 100)
+    params = [torch.nn.Parameter(torch.arange(60, dtype=torch.float32).reshape(6, 10)), torch.nn.Parameter(-torch.arange(90.0))]
+    for p in params:
+        p.grad = 2 * p.detach()
+    pred, loss = torch.randn(1, 2, 4, 8, 8, dtype=torch.bfloat16), torch.tensor(0.25)
+    runs = []
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), pred, loss, params)
+        runs.append({f.stem: np.load(f) for f in (tmp_path / d).iterdir()})
+    a, b = runs
+    assert sorted(a) == ["grads_sample", "loss", "pred", "sample_index", "weights_sample"]
+    for k in a:
+        assert a[k].dtype in (np.float32, np.float64) and np.array_equal(a[k], b[k]), k
+    idx = a["sample_index"].astype(np.int64)
+    flat = np.concatenate([p.detach().numpy().reshape(-1) for p in params])
+    assert 0 < len(idx) <= 100 and np.all(np.diff(idx) > 0) and idx[-1] < flat.size
+    assert np.array_equal(a["weights_sample"], flat[idx]) and np.array_equal(a["grads_sample"], 2 * flat[idx])
+    assert a["pred"].shape == (1, 2, 4, 8, 8) and np.array_equal(a["pred"], pred.float().numpy()) and a["loss"] == 0.25
+
+
 def test_splitk_workspace_is_cached_per_shape():
     from svd_xtend_b200 import raw
     import torch

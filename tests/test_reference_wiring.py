@@ -1,14 +1,14 @@
 """The oracle's (and the product class's) top-level wiring against the REFERENCE'S OWN file.
 
-tests/golden/ref_wiring_tiny.pt was produced by importing /root/reference/src/unet_spatio_temporal_condition.py unmodified
+tests/golden/ref_wiring_tiny.pt was produced by importing the reference's src/unet_spatio_temporal_condition.py unmodified
 (tests/golden/make_ref_wiring_golden.py, through oracle/ref_wiring.py) and running it in fp64 on two clips. These CPU tests
-need only the committed fixture; where /root/reference exists (the build container) the live A/B runs as well.
+need only the committed fixture.
 What is pinned: construction (:71-246), forward wiring (:357-490), plugin-API key set (:248-274), parameter census of the SVD
-configuration. The arithmetic inside the blocks is the oracle's on both sides (unpinned against diffusers)."""
+configuration, the gradients of one training-mode step. The arithmetic inside the blocks is the oracle's on both sides
+(unpinned against diffusers)."""
 import hashlib
 import importlib.util
 import os
-import sys
 
 import pytest
 import torch
@@ -68,40 +68,34 @@ def test_product_class_plugin_keys_equal_reference_file(gold):
     assert [(k, tuple(v.shape)) for k, v in m.state_dict().items()] == gold["tiny_keys"]
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/src/unet_spatio_temporal_condition.py"), reason="the reference checkout is not on this box")
 def test_live_reference_file_vs_oracle(gold):
-    """build container only: re-run the reference file itself and compare with the oracle and with the fixture"""
-    from oracle.ref_wiring import load_reference_unet_class
-    from oracle.svd_unet_oracle import UNetSpatioTemporalConditionModel as Oracle
-    sha = hashlib.sha256(open("/root/reference/src/unet_spatio_temporal_condition.py", "rb").read()).hexdigest()
-    assert sha == gold["reference_file_sha256"], "the fixture was generated from a different reference file"
+    """one training-mode step of the oracle against the same step of the reference file, as the fixture recorded it:
+    initial state dict, output, loss and every trainable gradient (fp64 on both sides: round-off only), plus the
+    reference's gradient-checkpointing hook and its plugin-API error on a mismatched processor dict"""
+    from oracle.svd_unet_oracle import TINY_CONFIG, UNetSpatioTemporalConditionModel as Oracle
+    from svd_xtend_b200.unet import UNetSpatioTemporalConditionModel as Ours
     gen = _gen()
-    Ref = load_reference_unet_class("/root/reference")
-    ref, ora = gen.build(Ref), gen.build(Oracle)
-    for (ka, va), (kb, vb) in zip(ref.state_dict().items(), ora.state_dict().items()):
-        assert ka == kb and torch.equal(va, vb)
-    b = gen.batch()
-    ref.train(), ora.train()
-    for m in (ref, ora):
-        m.requires_grad_(False)
-        for n, p in m.named_parameters():
-            if "temporal_transformer_block" in n:
-                p.requires_grad_(True)
-    outs = []
-    for m in (ref, ora):
-        out = m(b["sample"], b["timestep"].double(), b["encoder_hidden_states"], b["added_time_ids"]).sample
-        out.square().mean().backward()
-        outs.append(out.detach())
-    assert torch.equal(outs[0], outs[1])
-    assert ((outs[0] - gold["tiny_out"]).norm() / gold["tiny_out"].norm()).item() < 1e-12
-    for (n, p), (_, q) in zip(ref.named_parameters(), ora.named_parameters()):
-        if p.requires_grad:
-            assert torch.equal(p.grad, q.grad), n
-    # the plugin API of the reference file on the oracle's Attention modules
-    ref.set_default_attn_processor()
-    assert {type(p).__name__ for p in ref.attn_processors.values()} == {"AttnProcessor"}
-    with pytest.raises(ValueError):
-        ref.set_attn_processor({})
-    ref.enable_gradient_checkpointing()
-    assert sum(bool(getattr(m, "gradient_checkpointing", False)) for m in ref.modules()) == \
-        sum(1 for m in ora.modules() if hasattr(m, "gradient_checkpointing"))
+    ora = gen.build(Oracle)
+    sums = gen.state_sums(ora)
+    assert list(sums) == list(gold["train_state_sums"])
+    for k, (s, a) in gold["train_state_sums"].items():
+        assert abs(sums[k][0] - s) <= 1e-12 * a and abs(sums[k][1] - a) <= 1e-12 * a, k
+    out, loss = gen.train_step(ora, gen.batch())
+    assert ((out - gold["tiny_out"]).norm() / gold["tiny_out"].norm()).item() < 1e-12
+    assert abs(float(loss) - gold["train_loss"]) < 1e-12 * gold["train_loss"]
+    trainable = {n: p for n, p in ora.named_parameters() if p.requires_grad}
+    assert sorted(trainable) == sorted(list(gold["train_grads"]) + gold["train_zero_grads"])
+    for n in gold["train_zero_grads"]:
+        assert float(trainable[n].grad.abs().max()) == 0.0, n
+    for n, rec in gold["train_grads"].items():
+        g = trainable[n].grad.reshape(-1)
+        assert torch.equal(gen.grad_sample_index(g.numel()), rec["idx"]), n
+        assert abs(float(g.norm()) - rec["norm"]) <= 1e-10 * rec["norm"], n
+        assert (g[rec["idx"]] - rec["val"]).abs().max().item() <= 1e-10 * rec["norm"], n
+    assert sum(1 for m in ora.modules() if hasattr(m, "gradient_checkpointing")) == gold["grad_ckpt_modules"]
+    ours = Ours(**TINY_CONFIG)
+    ours.enable_gradient_checkpointing()
+    assert sum(bool(getattr(m, "gradient_checkpointing", False)) for m in ours.modules()) == gold["grad_ckpt_modules"]
+    with pytest.raises(Exception) as err:
+        ours.set_attn_processor({})
+    assert type(err.value).__name__ == gold["set_attn_processor_mismatch_error"]
