@@ -131,7 +131,16 @@ typedef struct SvdxTapGemm {
   float* gnb_sum;
   int32_t gnb_rows;
   int32_t gnb_silu;
+  /* activation of the accumulator (SVDX_ACT_*), applied before the residual / scale step:
+   *   v = act(acc + bias + rowbias),  out = scales[0] * v + scales[1] * res1 + scales[2] * res2.
+   * SVDX_ACT_GELU replaces the F.gelu of CLIPMLP (transformers CLIPVisionModelWithProjection, loaded at train_svd.py:646 and run
+   * at :875) on fc1's output. Requires a bf16 output, no GEGLU, no gn_sum / gnb_* statistics; with split_k > 1 the activation
+   * belongs to the second pass (svdx_splitk_epilogue_act). Zero (the default of a zero-initialised descriptor) = none. */
+  int32_t act;
 } SvdxTapGemm;
+
+#define SVDX_ACT_NONE 0
+#define SVDX_ACT_GELU 1   /* gelu(x) = x * Phi(x), the erf form (hidden_act "gelu") */
 
 int svdx_tapgemm(const SvdxTapGemm* desc, void* stream);
 
@@ -143,6 +152,12 @@ int svdx_tapgemm(const SvdxTapGemm* desc, void* stream);
 int svdx_splitk_epilogue(float* ws, int64_t ldw, void* out, int64_t ldo, int64_t rows, int32_t cols, const float* bias,
                          const float* rowbias, int32_t rowbias_div, int64_t ldrb, const void* res1, int64_t ldr1,
                          const void* res2, int64_t ldr2, const float* scales, void* stream);
+/* the same second pass with an activation (SVDX_ACT_*) applied before the residual step:
+ *   out = scales[0] * act(ws + bias + rowbias) + scales[1] * res1 + scales[2] * res2.
+ * Used for CLIPMLP.fc1 + F.gelu (train_svd.py:875 -> transformers CLIPMLP) at B = 1, where the 257-row GEMM has 3 row tiles. */
+int svdx_splitk_epilogue_act(float* ws, int64_t ldw, void* out, int64_t ldo, int64_t rows, int32_t cols, const float* bias,
+                             const float* rowbias, int32_t rowbias_div, int64_t ldrb, const void* res1, int64_t ldr1,
+                             const void* res2, int64_t ldr2, const float* scales, int32_t act, void* stream);
 
 /* number of SMs the persistent kernels size their grids to (queried once) */
 int svdx_num_sms(void);
@@ -155,7 +170,8 @@ int svdx_enable_peer_access(int32_t peer_device);
  * allocation can be imported once per process; the mapping lives until the process exits. */
 int svdx_ipc_export(const void* ptr, void* handle64_out, int64_t* offset_out);
 int svdx_ipc_import(const void* handle64, int64_t offset, void** ptr_out);
-/* sizeof(SvdxTapGemm) (which==0) / sizeof(SvdxAttn) (which==1): lets bindings verify their struct layout */
+/* sizeof(SvdxTapGemm) (which==0) / sizeof(SvdxAttn) (which==1) / sizeof(SvdxClipPixels) (which==2): lets bindings verify
+ * their struct layout */
 int svdx_struct_size(int which);
 /* human-readable last error of this thread */
 const char* svdx_last_error(void);
@@ -243,6 +259,42 @@ typedef struct SvdxAttn {
 } SvdxAttn;
 int svdx_attention_fwd(const SvdxAttn* d, void* stream);
 int svdx_attention_bwd(const SvdxAttn* d, void* stream);
+/* ViT self-attention of the CLIP image encoder, forward only: head_dim 80 (head h = columns [h*80, h*80+80), 160-byte
+ * offsets), no mask, 1 <= S <= 512 tokens per sequence (257 for ViT-H/14), sequences are contiguous blocks of rows
+ * (inner = 1, tok_stride = 1, outer_stride >= S; nseq = images). q / k / v may be column slices of one fused [tokens][3C]
+ * q|k|v matrix; o is written at the same head columns only. lse / backward fields are ignored. One launch per layer, no S x S
+ * matrix in memory. Replaces CLIPAttention's softmax(q k^T * scale) v (transformers, reached from train_svd.py:875). */
+int svdx_attention_vit_fwd(const SvdxAttn* d, void* stream);
+
+/* ------------------------------------------------------------------ CLIP image preprocessing
+ * svdx_clip_pixels: [B][3][H][W] images (NCHW contiguous, dtype code 0/1/2) -> the bf16 patch matrix of the ViT patch
+ * embedding, [B * 256][ldo] with row b * 256 + py * 16 + px holding the 3 * 14 * 14 = 588 values of patch (py, px) in
+ * (c, ky, kx) order (= patch_embedding.weight.view(C, 588)), columns 588 .. 591 zero (ldo >= 592, ldo % 8 == 0).
+ *   resize = 1 (encode_image, train_svd.py:857-876): separable Gaussian blur (taps wy[ky] / wx[kx], odd sizes <= 31, reflect
+ *              padding of (k - 1) / 2, as _gaussian_blur2d / _filter2d, train_svd.py:193-248), then bicubic align_corners=True
+ *              resampling to 224 x 224 (A = -0.75, source index dst * (in - 1) / 223, neighbours clamped: F.interpolate of
+ *              _resize_with_antialiasing, train_svd.py:140-167), then (x + 1) / 2 and (x - mean[c]) / std[c]
+ *              (CLIPImageProcessor(do_normalize=True, ...), train_svd.py:864-871). The host computes the taps per (H, W).
+ *              The arithmetic is float64 end to end (taps, source coordinates, cubic weights, sums, normalisation), so the
+ *              bf16 result is the correctly rounded value of the exact resize up to ties: in float32 the source coordinate
+ *              dst * (in - 1) / 223 alone carries ~1e-4 of error at the far edge, and cancellation around the mean leaves
+ *              values near zero with few correct bits. 14 <= H, 14 <= W <= 6144.
+ *   resize = 0 (CLIPVisionModelWithProjection(pixel_values)): H = W = 224, already normalised: patchify only.
+ * Replaces ~10 torch ops and the image processor's host round trip with one launch. */
+#define SVDX_CLIP_MAX_TAPS 31
+typedef struct SvdxClipPixels {
+  const void* x;
+  int32_t dtype;        /* 0 fp32, 1 bf16, 2 fp16 */
+  int32_t B, H, W;
+  int32_t resize;
+  int32_t ky, kx;       /* blur taps along H / W (resize = 1) */
+  double wy[SVDX_CLIP_MAX_TAPS];
+  double wx[SVDX_CLIP_MAX_TAPS];
+  double mean[3], std[3];
+  void* out;
+  int64_t ldo;
+} SvdxClipPixels;
+int svdx_clip_pixels(const SvdxClipPixels* d, void* stream);
 
 /* ------------------------------------------------------------------ elementwise / layout */
 /* weights -> bf16, optionally re-laid-out. src_bf16 is the SOURCE DTYPE CODE used by every entry of this section:

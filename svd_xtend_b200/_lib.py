@@ -17,6 +17,8 @@ LIB_PATH = Path(os.environ["SVDX_LIB"]) if os.environ.get("SVDX_LIB") else PKG /
 SVDX_MAX_TAPS = 27
 A_ROWS, A_CONV2D = 0, 1
 OUT_BF16, OUT_F32, OUT_F32_ATOMIC = 0, 1, 2
+ACT_NONE, ACT_GELU = 0, 1
+SVDX_CLIP_MAX_TAPS = 31
 
 c_void_p, c_int, c_i64, c_float = C.c_void_p, C.c_int32, C.c_int64, C.c_float
 
@@ -38,6 +40,7 @@ class SvdxTapGemm(C.Structure):
         ("gn_sum", c_void_p), ("gn_ld", c_i64), ("gn_rows", c_int),
         ("gnb_x", c_void_p), ("gnb_ldx", c_i64), ("gnb_x2", c_void_p), ("gnb_ldx2", c_i64), ("gnb_c1", c_int),
         ("gnb_ab", c_void_p), ("gnb_sum", c_void_p), ("gnb_rows", c_int), ("gnb_silu", c_int),
+        ("act", c_int),
     ]
 
 
@@ -55,10 +58,22 @@ class SvdxAttn(C.Structure):
     ]
 
 
+class SvdxClipPixels(C.Structure):
+    _fields_ = [
+        ("x", c_void_p), ("dtype", c_int), ("B", c_int), ("H", c_int), ("W", c_int), ("resize", c_int),
+        ("ky", c_int), ("kx", c_int),
+        ("wy", C.c_double * SVDX_CLIP_MAX_TAPS), ("wx", C.c_double * SVDX_CLIP_MAX_TAPS),
+        ("mean", C.c_double * 3), ("std", C.c_double * 3),
+        ("out", c_void_p), ("ldo", c_i64),
+    ]
+
+
 _PROTOS = {
     "svdx_tapgemm": [C.POINTER(SvdxTapGemm), c_void_p],
     "svdx_splitk_epilogue": [c_void_p, c_i64, c_void_p, c_i64, c_i64, c_int, c_void_p, c_void_p, c_int, c_i64, c_void_p, c_i64,
                              c_void_p, c_i64, c_void_p, c_void_p],
+    "svdx_splitk_epilogue_act": [c_void_p, c_i64, c_void_p, c_i64, c_i64, c_int, c_void_p, c_void_p, c_int, c_i64, c_void_p, c_i64,
+                                 c_void_p, c_i64, c_void_p, c_int, c_void_p],
     "svdx_num_sms": [],
     "svdx_enable_peer_access": [c_int],
     "svdx_ipc_export": [c_void_p, c_void_p, c_void_p],
@@ -83,6 +98,8 @@ _PROTOS = {
                            c_void_p, c_i64, c_void_p, c_i64, c_void_p, c_void_p, c_void_p],
     "svdx_attention_fwd": [C.POINTER(SvdxAttn), c_void_p],
     "svdx_attention_bwd": [C.POINTER(SvdxAttn), c_void_p],
+    "svdx_attention_vit_fwd": [C.POINTER(SvdxAttn), c_void_p],
+    "svdx_clip_pixels": [C.POINTER(SvdxClipPixels), c_void_p],
     "svdx_prep_weight": [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p],
     "svdx_unprep_conv_grad": [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p],
     "svdx_dot_diff": [c_void_p, c_void_p, c_void_p, c_i64, c_void_p, c_void_p],
@@ -139,7 +156,8 @@ def load() -> C.CDLL:
             fn = getattr(lib, name)
             fn.argtypes = args
             fn.restype = C.c_int
-        if lib.svdx_struct_size(0) != C.sizeof(SvdxTapGemm) or lib.svdx_struct_size(1) != C.sizeof(SvdxAttn):
+        if (lib.svdx_struct_size(0) != C.sizeof(SvdxTapGemm) or lib.svdx_struct_size(1) != C.sizeof(SvdxAttn)
+                or lib.svdx_struct_size(2) != C.sizeof(SvdxClipPixels)):
             raise RuntimeError("svd_xtend_b200: ctypes struct layout does not match the C ABI")
         lib.svdx_last_error.restype = C.c_char_p
         lib.svdx_last_error.argtypes = []

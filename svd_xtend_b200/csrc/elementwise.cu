@@ -386,12 +386,12 @@ __global__ void silu_bwd_f32_kernel(const float* __restrict__ x, const float* __
   if (i < n) dx[i] = dy[i] * silu_grad_f(x[i]);
 }
 
-// epilogue of a split-K contraction: out = s0*(ws + bias + rowbias[m/div]) + s1*res1 + s2*res2  (bf16), 8 columns per thread
+// epilogue of a split-K contraction: out = s0*act(ws + bias + rowbias[m/div]) + s1*res1 + s2*res2  (bf16), 8 columns per thread
 __global__ void __launch_bounds__(256) splitk_epilogue_kernel(float* __restrict__ ws, long long ldw, bf16* __restrict__ out, long long ldo,
                                                               long long rows, int cols, const float* __restrict__ bias,
                                                               const float* __restrict__ rowbias, int rb_div, long long ldrb,
                                                               const bf16* __restrict__ res1, long long ldr1, const bf16* __restrict__ res2,
-                                                              long long ldr2, const float* __restrict__ scales) {
+                                                              long long ldr2, const float* __restrict__ scales, int act) {
   const int cv = cols / 8;
   const long long idx = gtid();
   if (idx >= rows * cv) return;
@@ -413,6 +413,10 @@ __global__ void __launch_bounds__(256) splitk_epilogue_kernel(float* __restrict_
     const float* rb = rowbias + (r / rb_div) * ldrb + c;
 #pragma unroll
     for (int k = 0; k < 8; ++k) f[k] += rb[k];
+  }
+  if (act == SVDX_ACT_GELU) {
+#pragma unroll
+    for (int k = 0; k < 8; ++k) f[k] = gelu_erf_f(f[k]);
   }
 #pragma unroll
   for (int k = 0; k < 8; ++k) f[k] *= s0;
@@ -1036,15 +1040,22 @@ extern "C" int svdx_silu_bwd_f32(const float* x, const float* dy, float* dx, int
   return SVDX_OK;
 }
 
-extern "C" int svdx_splitk_epilogue(float* ws, int64_t ldw, void* out, int64_t ldo, int64_t rows, int32_t cols, const float* bias,
-                                    const float* rowbias, int32_t rowbias_div, int64_t ldrb, const void* res1, int64_t ldr1,
-                                    const void* res2, int64_t ldr2, const float* scales, void* stream) {
+extern "C" int svdx_splitk_epilogue_act(float* ws, int64_t ldw, void* out, int64_t ldo, int64_t rows, int32_t cols, const float* bias,
+                                        const float* rowbias, int32_t rowbias_div, int64_t ldrb, const void* res1, int64_t ldr1,
+                                        const void* res2, int64_t ldr2, const float* scales, int32_t act, void* stream) {
   if (!ws || !out || rows <= 0 || cols <= 0 || cols % 8 || ldw % 4 || ldo % 8 || (res1 && ldr1 % 8) || (res2 && ldr2 % 8) ||
-      (rowbias && rowbias_div <= 0))
+      (rowbias && rowbias_div <= 0) || (act != SVDX_ACT_NONE && act != SVDX_ACT_GELU))
     return svdx_fail(SVDX_E_BADARG, "splitk_epilogue: bad arguments");
   splitk_epilogue_kernel<<<nblocks(rows * (cols / 8)), 256, 0, ST(stream)>>>(ws, ldw, reinterpret_cast<bf16*>(out), ldo, rows, cols, bias, rowbias,
                                                                             rowbias_div, ldrb, reinterpret_cast<const bf16*>(res1), ldr1,
-                                                                            reinterpret_cast<const bf16*>(res2), ldr2, scales);
+                                                                            reinterpret_cast<const bf16*>(res2), ldr2, scales, act);
   SVDX_CHECK_LAUNCH("splitk_epilogue");
   return SVDX_OK;
+}
+
+extern "C" int svdx_splitk_epilogue(float* ws, int64_t ldw, void* out, int64_t ldo, int64_t rows, int32_t cols, const float* bias,
+                                    const float* rowbias, int32_t rowbias_div, int64_t ldrb, const void* res1, int64_t ldr1,
+                                    const void* res2, int64_t ldr2, const float* scales, void* stream) {
+  return svdx_splitk_epilogue_act(ws, ldw, out, ldo, rows, cols, bias, rowbias, rowbias_div, ldrb, res1, ldr1, res2, ldr2, scales,
+                                  SVDX_ACT_NONE, stream);
 }

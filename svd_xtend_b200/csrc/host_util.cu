@@ -140,5 +140,5 @@ int svdx_make_tmap(CUtensorMap* out, const void* base, int rank, const uint64_t*
 }
 
 extern "C" int svdx_struct_size(int which) {
-  return which == 0 ? (int)sizeof(SvdxTapGemm) : which == 1 ? (int)sizeof(SvdxAttn) : -1;
+  return which == 0 ? (int)sizeof(SvdxTapGemm) : which == 1 ? (int)sizeof(SvdxAttn) : which == 2 ? (int)sizeof(SvdxClipPixels) : -1;
 }

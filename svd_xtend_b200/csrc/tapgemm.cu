@@ -363,6 +363,8 @@ int svdx_tapgemm_fill(const SvdxTapGemm* d, TapGemmKParams& p, int cg) {
   if ((reinterpret_cast<uintptr_t>(d->a) & 15) || (reinterpret_cast<uintptr_t>(d->b) & 15)) return svdx_fail(SVDX_E_BADARG, "tapgemm: operands must be 16 B aligned");
   if ((d->a_major_mn || d->b_major_mn) && (d->a_mode != SVDX_A_ROWS || d->num_taps != 1)) return svdx_fail(SVDX_E_BADARG, "tapgemm: MN-major operands only in single-tap ROWS mode");
   if (d->b_mode != 0 && !(d->a_major_mn && d->b_major_mn)) return svdx_fail(SVDX_E_BADARG, "tapgemm: b_mode needs MN-major A and B (weight-gradient form)");
+  if (d->act != SVDX_ACT_NONE && (d->act != SVDX_ACT_GELU || d->geglu || d->gn_sum || d->gnb_sum || d->gnb_x || d->out_dtype != SVDX_OUT_BF16))
+    return svdx_fail(SVDX_E_BADARG, "tapgemm: act needs a bf16 output and no GEGLU / gn_sum / gnb_* statistics (split-K: svdx_splitk_epilogue_act)");
 
   memset(&p, 0, sizeof(p));
   p.a_mode = d->a_mode; p.a_mn = d->a_major_mn; p.b_mn = d->b_major_mn;
@@ -480,6 +482,7 @@ int svdx_tapgemm_fill(const SvdxTapGemm* d, TapGemmKParams& p, int cg) {
   p.gnb_x = reinterpret_cast<const bf16*>(d->gnb_x); p.gnb_ldx = d->gnb_ldx; p.gnb_c1 = d->gnb_x2 ? d->gnb_c1 : d->N;
   p.gnb_x2 = reinterpret_cast<const bf16*>(d->gnb_x2); p.gnb_ldx2 = d->gnb_ldx2;
   p.gnb_ab = d->gnb_ab; p.gnb_sum = d->gnb_sum; p.gnb_rows = d->gnb_rows; p.gnb_silu = d->gnb_silu;
+  p.act = d->act;
   {
     static int probe = -1;
     if (probe < 0) { const char* e = getenv("SVDX_EPI_PROBE"); probe = e ? atoi(e) : 0; }

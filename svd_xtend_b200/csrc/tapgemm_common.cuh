@@ -67,6 +67,7 @@ struct __align__(64) TapGemmKParams {
   const float* gnb_ab; // [slab][2][N]: forward scale / shift per channel (y = act(x * scale + shift))
   float* gnb_sum;      // [slab][2][N], zero on entry: sum(e), sum(e * x), e = dy * act'(x * scale + shift)
   int gnb_rows, gnb_silu;
+  int act;             // SVDX_ACT_*: activation of acc + bias + rowbias, before residuals / scales
   int tma_store;       // epilogue stores through shared memory + TMA (tmo / tmpre valid)
   int epi_mode;        // EPI_GENERIC / EPI_FAST / EPI_GEGLU / EPI_RES: which kernel instantiation runs
   int probe;   // dev switch SVDX_EPI_PROBE: 1 = epilogue without global stores, 2 = no epilogue work at all
@@ -231,6 +232,14 @@ SVDX_DEVINL void stage_row_bf16(uint32_t row, int sw, const float (&f)[32]) {
                  pack_bf16x2(f[8 * j + 4], f[8 * j + 5]), pack_bf16x2(f[8 * j + 6], f[8 * j + 7]));
 }
 
+// activation of one 32-column chunk (p.act, warp-uniform)
+SVDX_DEVINL void act32(float (&f)[32], int act) {
+  if (act == SVDX_ACT_GELU) {
+#pragma unroll
+    for (int i = 0; i < 32; ++i) f[i] = gelu_erf_f(f[i]);
+  }
+}
+
 // Epilogue operands that are read per chunk (the residual of EPI_RES, the GroupNorm input of EPI_FAST_GNB) are usually not in L2
 // any more; a warp has ONE chunk's loads in flight, so the fetch was latency-bound (+12 us on a 15 us K = 320 residual GEMM,
 // +20 us on a conv dgrad with the backward sums). Each epilogue warp therefore requests its 32 rows x bn columns of the tile
@@ -282,6 +291,7 @@ SVDX_DEVINL void epilogue_fast(const TapGemmKParams& p, uint32_t t_base, long lo
     for (int i = 0; i < 32; ++i) { fa[i] = __uint_as_float(va[i]); fb[i] = __uint_as_float(vb[i]); }
     if (bias) { add_vec32(fa, bias + colA); if (hasB) add_vec32(fb, bias + colB); }
     if (rb) { add_vec32(fa, rb + colA); if (hasB) add_vec32(fb, rb + colB); }
+    if (p.act) { act32(fa, p.act); if (hasB) act32(fb, p.act); }
     if (lane == 0) bulk_wait_read<0>();   // the previous round's stores have drained both halves
     __syncwarp();
     stage_row_bf16(rowX, sw, fa);
@@ -472,6 +482,7 @@ SVDX_DEVINL void epilogue_res(const TapGemmKParams& p, uint32_t t_base, long lon
     for (int i = 0; i < 32; ++i) f[i] = __uint_as_float(v[i]);
     if (bias) add_vec32(f, bias + col0);
     if (rb) add_vec32(f, rb + col0);
+    if (p.act) act32(f, p.act);
     if (scaled) {
 #pragma unroll
       for (int i = 0; i < 32; ++i) f[i] *= s_acc;
@@ -673,6 +684,7 @@ SVDX_DEVINL void epilogue_tile(const TapGemmKParams& p, uint32_t t_base, long lo
               if (full_chunk || col0 + i < n_out_total) f[i] += __ldg(rb + col0 + i);
           }
         }
+        if (p.act) act32(f, p.act);
         if (p.scales) {
 #pragma unroll
           for (int i = 0; i < 32; ++i) f[i] *= s_acc;

@@ -379,10 +379,12 @@ class Engine:
     def linear(self, x: Var, weight, bias=None, *, res1: Optional[Var] = None, res2: Optional[Var] = None,
                scales: Optional[torch.Tensor] = None, res1_unit: bool = False, geglu: bool = False,
                rowbias: Optional[Var] = None, rowbias_div: int = 1, out_f32: bool = False,
-               fused: Optional[Sequence] = None, blend=None, lora: Optional[Sequence] = None, gn_rows: Optional[int] = None) -> Var:
+               fused: Optional[Sequence] = None, blend=None, lora: Optional[Sequence] = None, gn_rows: Optional[int] = None,
+               act: int = raw.ACT_NONE) -> Var:
         """y = epilogue(x @ W^T). `weight` is a parameter [N,K] (or conv 1x1 [N,K,1,1]); `fused` = list of
         parameters whose rows are concatenated (q|k|v). scales (device float[>=3]) = {acc, res1, res2};
-        res1_unit: scales[1] is known to be exactly 1. rowbias: Var with fp32 data [ceil(M/div), N]."""
+        res1_unit: scales[1] is known to be exactly 1. rowbias: Var with fp32 data [ceil(M/div), N].
+        act (raw.ACT_GELU): activation of acc + bias before the residual step; forward-only (no backward is recorded)."""
         ws = list(fused) if fused is not None else [weight]
         wf = self.w_lin_cat(ws, False) if fused is not None else self.w_lin(weight, False)
         N, K = wf.shape
@@ -392,10 +394,13 @@ class Engine:
         pre = self.empty(M, N, x.data) if (geglu and self.recording) else None
         b32 = self.vec_f32(bias)
         lora = [l for l in (lora or []) if l is not None]
-        sink = None if (geglu or out_f32 or lora) else self._gn_sink(gn_rows, M, N, K, 1, out.device)
+        if act and (geglu or out_f32 or lora):
+            raise ValueError("Engine.linear: act needs a plain bf16 linear (no GEGLU, fp32 output or LoRA)")
+        sink = None if (geglu or out_f32 or lora or act) else self._gn_sink(gn_rows, M, N, K, 1, out.device)
         raw.tapgemm_auto(x.data, wf, out, M=M, N=N, K=K, bias=b32, res1=None if res1 is None else res1.data,
                          res2=None if res2 is None else res2.data, scales=scales, geglu=geglu, pre=pre,
-                         rowbias=None if rowbias is None else rowbias.data, rowbias_div=rowbias_div, gn_sum=sink, gn_rows=gn_rows or 0)
+                         rowbias=None if rowbias is None else rowbias.data, rowbias_div=rowbias_div, gn_sum=sink, gn_rows=gn_rows or 0,
+                         act=act)
         lora_t = []
         for (off, n, A, Bm, sc) in lora:
             # LoRA side path (train_svd_lora.py:659-671): out[:, off:off+n] += scale * (x A^T) B^T, accumulated in place.
@@ -414,6 +419,8 @@ class Engine:
         w_train = any(p.requires_grad for p in ws) or (bias is not None and bias.requires_grad) \
             or (blend is not None and blend[0].requires_grad) or any(l[2].requires_grad or l[3].requires_grad for l in lora)
         need = x.needs_grad or w_train or any(v is not None and v.needs_grad for v in (res1, res2, rowbias))
+        if act and need and self.recording:
+            raise RuntimeError("Engine.linear: the activation epilogue is forward-only; it cannot record a backward")
         y = Var(out, need)
         if sink is not None:
             y.csum = (gn_rows, [(sink, N)])

@@ -2,13 +2,15 @@
 from __future__ import annotations
 
 import ctypes as C
+import functools
+import math
 import os
 from typing import Optional, Sequence
 
 import torch
 
 from . import _lib
-from ._lib import A_CONV2D, A_ROWS, OUT_BF16, OUT_F32, OUT_F32_ATOMIC, SvdxAttn, SvdxTapGemm, load
+from ._lib import A_CONV2D, A_ROWS, ACT_GELU, ACT_NONE, OUT_BF16, OUT_F32, OUT_F32_ATOMIC, SvdxAttn, SvdxClipPixels, SvdxTapGemm, load
 
 bf16 = torch.bfloat16
 
@@ -229,10 +231,12 @@ def tapgemm(
     gn_sum: Optional[torch.Tensor] = None,
     gn_rows: int = 0,
     gnb: Optional[dict] = None,
+    act: int = ACT_NONE,
 ) -> torch.Tensor:
     """Launch svdx_tapgemm on the current stream. All tensors are CUDA; a/b/res/pre are bf16.
     gn_sum: zeroed fp32 [slabs, 2, C] buffer that receives the per-channel sum / sum of squares of the output (fused
-    GroupNorm statistics), one slab per gn_rows output rows."""
+    GroupNorm statistics), one slab per gn_rows output rows.
+    act: activation of acc + bias + rowbias before the residual step (ACT_GELU: the erf GELU; bf16 output only)."""
     family = "conv" if (mode == A_CONV2D or len(taps) > 1 or b_mode != 0) else "linear"
     if _fam(family, 2.0 * M * N * K * len(taps)):
         return out
@@ -315,6 +319,7 @@ def tapgemm(
         d.gnb_sum = gnb["sum"].data_ptr()
         d.gnb_rows = gnb["rows"]
         d.gnb_silu = int(gnb["silu"])
+    d.act = int(act)
     check(load().svdx_tapgemm(C.byref(d), _stream()), "svdx_tapgemm")
     return out
 
@@ -351,15 +356,16 @@ def split_plan(out_is_bf16: bool, M: int, N: int, K: int, ntaps: int = 1, geglu=
 
 
 def tapgemm_auto(a, b, out, *, M, N, K, taps=((0, 0, 0),), bias=None, rowbias=None, rowbias_div=1, res1=None, res2=None,
-                 scales=None, gn_sum=None, gn_rows=0, **kw):
+                 scales=None, gn_sum=None, gn_rows=0, act=ACT_NONE, **kw):
     """svdx_tapgemm with automatic split-K for small-M / long-K problems (bf16 output, K-major operands, no GEGLU):
     when 128x256 tiles cannot fill the SMs, the contraction is split over CTAs (fp32 atomics into a workspace) and
-    svdx_splitk_epilogue applies bias / row-bias / residuals / scales. Fused GroupNorm statistics (gn_sum) exist on the
-    whole-problem path only: callers ask `split_plan` first and keep the stand-alone statistics kernel for split outputs."""
+    svdx_splitk_epilogue(_act) applies bias / row-bias / activation / residuals / scales. Fused GroupNorm statistics (gn_sum)
+    exist on the whole-problem path only: callers ask `split_plan` first and keep the stand-alone statistics kernel for split
+    outputs."""
     kw = dict(kw)
     if kw.get("block_n") is None:
         kw.pop("block_n", None)
-    if (M <= 8 and len(taps) == 1 and kw.get("mode", A_ROWS) == A_ROWS and not kw.get("geglu") and not kw.get("a_mn") and not kw.get("b_mn")
+    if (M <= 8 and not act and len(taps) == 1 and kw.get("mode", A_ROWS) == A_ROWS and not kw.get("geglu") and not kw.get("a_mn") and not kw.get("b_mn")
             and rowbias is None and res1 is None and res2 is None and scales is None and gn_sum is None and kw.get("groups", 1) == 1
             and K % 8 == 0 and a.stride(-1) == 1 and b.stride(-1) == 1 and out.dtype in (bf16, torch.float32)):
         # conditioning vectors ([B, C] rows): a GEMV, not a 128-row tensor-core tile
@@ -372,14 +378,24 @@ def tapgemm_auto(a, b, out, *, M, N, K, taps=((0, 0, 0),), bias=None, rowbias=No
         tapgemm(a, b, ws, M=M, N=N, K=K, taps=taps, block_n=bn, split_k=split, out_dtype=OUT_F32_ATOMIC, **kw)
         if _fam("conv" if (kw.get("mode", A_ROWS) == A_CONV2D or len(taps) > 1) else "linear"):
             return out
-        check(load().svdx_splitk_epilogue(ws.data_ptr(), N, out.data_ptr(), _rowmajor(out, "out"), M, N, _ptr(bias), _ptr(rowbias),
-                                          rowbias_div, _rowmajor(rowbias, "rowbias") if rowbias is not None else 0,
-                                          _ptr(res1), _rowmajor(res1, "res1") if res1 is not None else 0,
-                                          _ptr(res2), _rowmajor(res2, "res2") if res2 is not None else 0,
-                                          _ptr(scales), _stream()), "svdx_splitk_epilogue")
+        check(load().svdx_splitk_epilogue_act(ws.data_ptr(), N, out.data_ptr(), _rowmajor(out, "out"), M, N, _ptr(bias), _ptr(rowbias),
+                                              rowbias_div, _rowmajor(rowbias, "rowbias") if rowbias is not None else 0,
+                                              _ptr(res1), _rowmajor(res1, "res1") if res1 is not None else 0,
+                                              _ptr(res2), _rowmajor(res2, "res2") if res2 is not None else 0,
+                                              _ptr(scales), int(act), _stream()), "svdx_splitk_epilogue_act")
         return out
     return tapgemm(a, b, out, M=M, N=N, K=K, taps=taps, bias=bias, rowbias=rowbias, rowbias_div=rowbias_div, res1=res1, res2=res2,
-                   scales=scales, gn_sum=gn_sum, gn_rows=gn_rows, **kw)
+                   scales=scales, gn_sum=gn_sum, gn_rows=gn_rows, act=act, **kw)
+
+
+def fill_rows(out: torch.Tensor, vec: torch.Tensor) -> torch.Tensor:
+    """out[r, :] = bf16(vec) for every row of a bf16 [rows, N] view (any row stride): the split-K epilogue over its zeroed
+    workspace with vec (fp32 [N]) as the bias (the CLIP class-token rows, one launch for the whole batch)"""
+    rows, N = out.shape
+    ws = _splitk_workspace(rows, N, out.device)
+    check(load().svdx_splitk_epilogue_act(ws.data_ptr(), N, out.data_ptr(), _rowmajor(out, "out"), rows, N, vec.data_ptr(), None, 1, 0,
+                                          None, 0, None, 0, None, ACT_NONE, _stream()), "svdx_splitk_epilogue_act")
+    return out
 
 
 CONV3x3_TAPS = tuple((kw - 1, kh - 1, 0) for kh in range(3) for kw in range(3))
@@ -406,6 +422,16 @@ def attention_fwd(q, k, v, o, *, heads, S, nseq, inner=1, outer_stride=None, inn
         return o
     d = _attn_desc(q, k, v, o, heads, S, nseq, inner, outer_stride, inner_stride, tok_stride, scale, lse)
     check(load().svdx_attention_fwd(C.byref(d), _stream()), "svdx_attention_fwd")
+    return o
+
+
+def attention_vit(q, k, v, o, *, heads, S, nseq, scale=80 ** -0.5):
+    """ViT self-attention, head_dim 80, forward only (svdx_attention_vit_fwd): q/k/v/o [nseq * S, >= heads*80] bf16 column
+    slices (q, k, v usually of one fused [rows, 3C] q|k|v matrix); sequence s = rows [s*S, (s+1)*S)"""
+    if _fam("attention", 4.0 * nseq * heads * S * S * 80):
+        return o
+    d = _attn_desc(q, k, v, o, heads, S, nseq, 1, S, 0, 1, scale, None)
+    check(load().svdx_attention_vit_fwd(C.byref(d), _stream()), "svdx_attention_vit_fwd")
     return o
 
 
@@ -516,6 +542,60 @@ def layernorm_bwd(x, dy, gamma, mean, rstd, dx, dres=None, dgamma=None, dbeta=No
                                     mean.data_ptr(), rstd.data_ptr(), dx.data_ptr(), _rowmajor(dx, "dx"), _ptr(dres),
                                     _rowmajor(dres, "dres") if dres is not None else 0, _ptr(dgamma), _ptr(dbeta), _stream()),
           "layernorm_bwd")
+
+
+# ----------------------------------------------------------------------------- CLIP preprocessing
+CLIP_SIZE = 224
+CLIP_PATCH_K = 588       # 3 x 14 x 14 values of one patch
+CLIP_PATCH_KP = 592      # padded to 16-byte rows
+
+
+@functools.lru_cache(maxsize=None)
+def clip_blur_taps(H: int, W: int):
+    """(ky, kx, wy, wx, (sigma_y, sigma_x)) of the anti-aliasing blur applied before resampling an H x W image to 224 x 224
+    (train_svd.py:140-162, 218-232): sigma = max((in / 224 - 1) / 2, 0.001) per axis, kernel size int(max(4 sigma, 3)) made
+    odd, normalised Gaussian taps computed in float64"""
+    sig = tuple(max((n / CLIP_SIZE - 1.0) / 2.0, 0.001) for n in (H, W))
+    ks = []
+    for s in sig:
+        k = int(max(2.0 * 2 * s, 3))
+        ks.append(k + 1 if k % 2 == 0 else k)
+    taps = []
+    for k, s in zip(ks, sig):
+        g = [math.exp(-float(i - k // 2) ** 2 / (2.0 * s * s)) for i in range(k)]
+        tot = math.fsum(g)
+        taps.append(tuple(v / tot for v in g))
+    return ks[0], ks[1], taps[0], taps[1], sig
+
+
+def clip_pixels(x: torch.Tensor, out: torch.Tensor, *, resize: bool, mean=(0.0, 0.0, 0.0), std=(1.0, 1.0, 1.0)) -> torch.Tensor:
+    """[B, 3, H, W] images -> bf16 patch matrix out [B*256, >= 592] (svdx_clip_pixels). resize=True: anti-aliased bicubic
+    resize to 224 x 224, (x + 1) / 2, (x - mean) / std; resize=False: an already normalised 224 x 224 input, patchify only."""
+    B, Cc, H, W = x.shape
+    if Cc != 3 or not x.is_contiguous():
+        raise ValueError("clip_pixels: x must be a contiguous [B, 3, H, W] tensor")
+    if out.dtype != bf16 or out.dim() != 2 or out.shape[0] != B * 256 or out.shape[1] < CLIP_PATCH_KP:
+        raise ValueError("clip_pixels: out must be a bf16 [B * 256, >= 592] matrix")
+    d = SvdxClipPixels()
+    d.x = x.data_ptr()
+    d.dtype = dtype_code(x, "image")
+    d.B, d.H, d.W = B, H, W
+    d.resize = int(resize)
+    if resize:
+        ky, kx, wy, wx, _ = clip_blur_taps(H, W)
+        if max(ky, kx) > _lib.SVDX_CLIP_MAX_TAPS:
+            raise ValueError(f"clip_pixels: {H}x{W} needs a {ky}x{kx} blur; at most {_lib.SVDX_CLIP_MAX_TAPS} taps per axis are supported")
+        d.ky, d.kx = ky, kx
+        for i, v in enumerate(wy):
+            d.wy[i] = v
+        for i, v in enumerate(wx):
+            d.wx[i] = v
+    for i in range(3):
+        d.mean[i], d.std[i] = float(mean[i]), float(std[i])
+    d.out = out.data_ptr()
+    d.ldo = _rowmajor(out, "out")
+    check(load().svdx_clip_pixels(C.byref(d), _stream()), "svdx_clip_pixels")
+    return out
 
 
 # ----------------------------------------------------------------------------- elementwise / layout

@@ -10,7 +10,9 @@ CUDA graph replays all `num_inference_steps` steps; between replays the host onl
 Scheduler constants follow diffusers' EulerDiscreteScheduler in the SVD configuration [D] (Karras sigmas, rho 7, sigma in
 [0.002, 700], timesteps 0.25 ln sigma, init_noise_sigma sqrt(sigma_max^2 + 1)); tests/test_sampling_gpu.py checks the loop
 against oracle/svd_sampling_oracle.py. Out of scope here: VAE encode / decode and the CLIP image encoder (SURVEY.md §8f-1/-4) —
-`image_latents` and `image_embeddings` are inputs, denoised latents are the output.
+`image_latents` and `image_embeddings` are inputs, denoised latents are the output. `image_embeddings` come from
+`svd_xtend_b200.clip.encode_image(frame, image_encoder)` (the conditioning frame in [-1, 1]), the VAE latents from
+`svd_xtend_b200.vae`.
 """
 from __future__ import annotations
 

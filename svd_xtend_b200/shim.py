@@ -5,7 +5,9 @@
 
 Before the script body runs, the replacement class is installed under the two names the reference
 imports the UNet from: `diffusers.UNetSpatioTemporalConditionModel` (train_svd.py:49) and
-`src.unet_spatio_temporal_condition.UNetSpatioTemporalConditionModel` (train_svd_lora.py:60).
+`src.unet_spatio_temporal_condition.UNetSpatioTemporalConditionModel` (train_svd_lora.py:60). When `transformers` is
+importable, the CLIP image encoder is also installed as `transformers.CLIPVisionModelWithProjection` (train_svd.py:43,
+train_svd_lora.py:43); the scripts' CLIPImageProcessor stays transformers' own.
 diffusers / accelerate are NOT part of this image (no network), so this shim is exercised only where a
 user's environment provides them; it fails loudly when they are missing.
 """
@@ -38,6 +40,19 @@ def install() -> None:
     sys.modules["src"] = pkg
     sys.modules["src.unet_spatio_temporal_condition"] = sub
     pkg.unet_spatio_temporal_condition = sub
+    install_clip()
+
+
+def install_clip() -> bool:
+    """install svd_xtend_b200.clip.CLIPVisionModelWithProjection as transformers.CLIPVisionModelWithProjection; False when
+    transformers is not importable (the scripts then fail on their own import, as before)"""
+    from .clip import CLIPVisionModelWithProjection
+    try:
+        transformers = importlib.import_module("transformers")
+    except ModuleNotFoundError:
+        return False
+    transformers.CLIPVisionModelWithProjection = CLIPVisionModelWithProjection
+    return True
 
 
 def main(argv=None) -> None:
